@@ -330,6 +330,8 @@ def run_b200(args, rank, world, local_rank):
     l0 = ctx.launches
     ms = timed(step, args.steps)
     launches = ctx.launches - l0
+    # the last timed step's outputs, copied on the device before the untimed steps below rewrite them
+    snapshot = [t.clone() for t in (d_sad, d_satd, d_best, d_best2, d_coef)] if args.dump_outputs and rank == 0 else None
     for _ in range(int(min(2000, max(0, 250.0 / max(ms / args.steps, 1e-3) - args.steps)))):   # ~0.25 s more of the
         step()                                                   # same steps (untimed): clock samples under load
     torch.cuda.synchronize()
@@ -481,8 +483,31 @@ def run_b200(args, rank, world, local_rank):
         }
         if tiles4k is not None:
             out["strong_scaling_4k_tiles"] = tiles4k
+        if snapshot is not None:
+            s_sad, s_satd, s_best, s_best2, s_coef = (t.cpu().numpy() for t in snapshot)
+            winners = lambda b: np.stack([b["cost"], b["sad"], b["mv_row"], b["mv_col"]], axis=1)
+            dump_outputs(args.dump_outputs, {
+                "sad_candidates": s_sad.view(np.uint32), "satd_candidates": s_satd.view(np.uint32),
+                "sad_winners": winners(s_best.view(B.ME_RESULT_DTYPE)),
+                "satd_winners": winners(s_best2.view(B.ME_RESULT_DTYPE)),
+                "coefficients": s_coef.reshape(F * nb, BW * BH)})
         print(json.dumps(out))
     finish(world, dist)
+
+
+DUMP_VALUES = 1 << 20      # values kept per output by --dump-outputs (8 MB as float64)
+
+
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: every output as out_dir/<name>.npy in float64, which holds all of their values exactly.  Rows
+    are the step's blocks or candidates, frame after frame.  An output of more than DUMP_VALUES values keeps a sample
+    of its rows, in order, drawn from a fixed seed: the same rows at every run with the same arguments."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        keep = max(1, DUMP_VALUES // (a.size // len(a)))
+        if len(a) > keep:
+            a = a[np.sort(np.random.default_rng(0).choice(len(a), keep, replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float64))
 
 
 def finish(world, dist):
@@ -841,7 +866,7 @@ def run_e2e_lists(ctx0, blocks, args, world=1, dist=None):
         h2d, d2h = sum(r[0] for r in res), sum(r[1] for r in res)
     for _ in range(2):
         step()
-    reps = max(3, min(args.steps, 10))
+    reps = args.steps
     l0 = sum(cx.launches for cx in ctxs)
     if world > 1:
         dist.barrier()
@@ -989,7 +1014,7 @@ def run_e2e_stream(ctx0, blocks, args, world=1, dist=None):
             tot[q] = sum(r[q] for r in res)
     for _ in range(2):
         step()
-    reps = max(3, min(args.steps, 10))
+    reps = args.steps
     l0 = sum(cx.launches for cx in ctxs)
     if world > 1:
         dist.barrier()
@@ -1097,7 +1122,14 @@ def main():
     ap.add_argument("--graph", action="store_true", help="4k-tiles at N > 1: capture the step (incl. the NCCL all-gather) in a CUDA graph")
     ap.add_argument("--pairs-per-launch", type=int, default=32,
                     help="frame pairs served by one launch of each leg (b200_*_multi_dev); 1 = a launch per pair")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last 1080p step computed on rank 0 as DIR/<name>.npy "
+                         "(float64, at most 64 MB in all): per-candidate SAD and SATD, the SAD and SATD winners "
+                         "(cost, distortion, mv_row, mv_col) and the winners' coefficients; the inputs are seeded, so "
+                         "runs with the same arguments compare output for output")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "b200" or args.workload == "4k-tiles"):
+        ap.error("--dump-outputs writes the outputs of the b200 arm's 1080p step (--impl b200, --workload auto or 1080p)")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

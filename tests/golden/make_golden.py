@@ -18,7 +18,8 @@ Sources (xiph/rav1e @ 564ae3b):
                                bytes and sha256 of each; the oracle and the CUDA side regenerate
                                them from their rule)
   tests/small_input.y4m   BASELINE config 0's input: the luma planes of its 5 frames (64x64, 8 bit)
-                          -> tests/golden/small_input_luma.npy
+                          -> tests/golden/small_input_luma.npy, and the clip itself (31 KB), byte for byte
+                          -> tests/golden/small_input.y4m, so that the Y4M reader is checked without rav1e
 The Rust test code is parsed textually; nothing is executed (no rustc in this image).
 """
 import json
@@ -118,6 +119,9 @@ def main():
     assert luma.shape == (5, 64, 64)
     np.save(os.path.join(os.path.dirname(OUT), "small_input_luma.npy"), luma)
     print("wrote small_input_luma.npy", luma.shape, int(luma.sum()))
+    with open(os.path.join(os.path.dirname(OUT), "small_input.y4m"), "wb") as f:
+        f.write(raw)
+    print("wrote small_input.y4m", len(raw), "bytes")
 
 
 if __name__ == "__main__":

@@ -1,6 +1,6 @@
 """examples/stream_frames.cpp is the C-ABI-only walk through the frame pipe (create, resident lists, one packed push
-per frame).  Here: it compiles and links against the shared library with nothing but the public header, and on a
-machine without a GPU it fails loudly instead of computing anything on the CPU."""
+per frame).  Here: it compiles and links against the shared library with nothing but the public header, with no
+CUDA device visible it fails loudly instead of computing anything on the CPU, and on a GPU it streams frames."""
 import os
 import subprocess
 
@@ -18,10 +18,15 @@ def build(tmp_path):
 
 
 def test_example_builds_and_refuses_to_run_without_a_gpu(tmp_path):
-    import torch
     exe = build(tmp_path)
-    if torch.cuda.is_available():
-        pytest.skip("GPU present: covered by the gpu-marked test")
-    r = subprocess.run([exe, "2"], capture_output=True, text=True)
+    # an empty CUDA_VISIBLE_DEVICES hides the devices of a GPU machine as well
+    r = subprocess.run([exe, "2"], capture_output=True, text=True, env=dict(os.environ, CUDA_VISIBLE_DEVICES=""))
     assert r.returncode != 0 and "no CPU fallback" in r.stderr
 
+
+@pytest.mark.gpu
+def test_example_streams_frames_on_the_gpu(tmp_path):
+    exe = build(tmp_path)
+    r = subprocess.run([exe, "3"], capture_output=True, text=True, timeout=300)
+    assert r.returncode == 0, r.stdout + r.stderr
+    assert r.stdout.startswith("3 frames in "), r.stdout
