@@ -4,6 +4,7 @@
 #include <cuda_runtime.h>
 
 #include <algorithm>
+#include <limits>
 #include <vector>
 
 #include "common.cuh"
@@ -43,6 +44,16 @@ __device__ __forceinline__ int dequant1(int c, uint32_t quant, int log_tx_scale)
   return (int)((uint32_t)c * quant + (uint32_t)((c >> 31) & offset)) >> log_tx_scale;
 }
 
+// `c.abs() >= deadzone` with c: T, quantize/mod.rs:296.  The reference's release build negates with
+// wrapping, so T::MIN.abs() is T::MIN and never reaches the deadzone.  Evaluated in 32 bits with T::MIN
+// singled out: a 16-bit abs of -32768 on the device yields +32768, which counted a -32768 coefficient
+// towards the end of block.
+template <typename T>
+__device__ __forceinline__ bool reaches_deadzone(T v, int deadzone) {
+  const int iv = (int)v;
+  return iv != (int)std::numeric_limits<T>::min() && (iv < 0 ? -iv : iv) >= deadzone;
+}
+
 // h(x) = after(before(x)) for functions {0,1} -> {0,1} stored as bit x = f(x)
 __device__ __forceinline__ uint32_t compose(uint32_t after, uint32_t before) {
   return ((after >> (before & 1)) & 1) | (((after >> ((before >> 1) & 1)) & 1) << 1);
@@ -62,8 +73,7 @@ __device__ __forceinline__ void quantize_block_warp(const QuantArgs &a, const T 
       const T v = c[i];
       ss += sq_i32((int)v);
       if (i < a.coded) {
-        const T av = (T)(v < 0 ? -v : v);
-        if (av >= (T)a.deadzone) em1 = max(em1, (uint32_t)a.iscan[i]);
+        if (reaches_deadzone(v, a.deadzone)) em1 = max(em1, (uint32_t)a.iscan[i]);
         q[i] = 0;
         if (r) r[i] = 0;
       }
