@@ -6,7 +6,9 @@
 // inter = px << ib exactly (128 px is a multiple of 2^(7-ib)), after which the V rounding
 // (sum + 2^(6+ib)) >> (7+ib) equals the V-only (sum + 64) >> 7; an identity V pass turns
 // round(128 * inter, 7+ib) into round(inter, ib), the H-only case's second rounding; and the i16
-// intermediate never truncates (|inter| <= 20.5 K at every bit depth).  So one code path serves all.
+// intermediate never truncates: over the filter table it lies in [-1785, 5865] at 8 bit, [-7161, 23529]
+// at 10 and [-7166, 23546] at 12 (tests/test_full_scale_pred.py computes and pins these bounds).  So one
+// code path serves all.
 //
 // Arithmetic on packed words instead of one multiply per tap and pixel:
 //   H pass, 8-bit pixels : IDP.4A - four u8 pixels x four s8 taps per instruction (every tap fits s8:
